@@ -8,9 +8,11 @@ One "step" = one pass of the hot path over one batch of synthetic queries.
   cpu_baseline / --impl reference : the restated reference algorithm (Block-max WAND, oracle/) on the host cores
 
 Launch: `python bench.py --gpus N --steps K --warmup W` (N>1: under torchrun, one rank per GPU; queries are
-sharded across ranks with the index replicated — weak scaling: every rank runs its own full batch).
+sharded across ranks with the index replicated — weak scaling: every rank runs its own full batch).  Every timed loop
+runs K steps.  `--dump-outputs DIR` writes the result rows of the last timed step as DIR/<name>.npy (dump_outputs()).
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -40,10 +42,17 @@ WORKLOADS = {
 }
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=positive_int, default=10, help="timed steps of every timed loop")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
@@ -54,6 +63,8 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling side leg of the default run")
     ap.add_argument("--no-prune", action="store_true", help="disable MaxScore-style pruning (exhaustive streaming)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's results of the last timed step as DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -72,6 +83,7 @@ class ClockSampler:
                                           "--format=csv,noheader,nounits", "-lms", "100"], stdout=subprocess.PIPE,
                                          stderr=subprocess.DEVNULL, text=True)
             threading.Thread(target=self._read, daemon=True).start()
+            atexit.register(self._end)   # a run that fails between start() and stop() must not leave nvidia-smi behind
         except Exception:
             self.proc = None
 
@@ -79,9 +91,13 @@ class ClockSampler:
         for line in self.proc.stdout:
             self.rows.append([x.strip() for x in line.split(",")])
 
-    def stop(self):
-        if self.proc:
+    def _end(self):
+        if self.proc and self.proc.poll() is None:
             self.proc.terminate()
+            self.proc.wait()
+
+    def stop(self):
+        self._end()
         sm = [float(r[1]) for r in self.rows if len(r) >= 8 and r[1].replace(".", "").isdigit()]
         mx = [float(r[2]) for r in self.rows if len(r) >= 8 and r[2].replace(".", "").isdigit()]
         reasons = set()
@@ -164,10 +180,37 @@ def cpu_reference(oix, q_off, q_terms, k, n, threads):
     return n / dt, n, dt, st
 
 
+DUMP_BYTES = 60_000_000  # --dump-outputs: array bytes in all (under 64 MB with the .npy headers)
+DUMP_SEED = 0xB25D0       # --dump-outputs: the row sample when all rows would not fit
+
+
+def dump_outputs(d, res):
+    """--dump-outputs: the result rows a caller of the timed path receives, as DIR/<name>.npy — doc ids and row counts
+    as float64 (exact), scores in their own precision (score f32, score64 f64).  Slots past a row's count n are not
+    defined by the C ABI and are written as 0.  When every row would take more than DUMP_BYTES, a fixed seeded sample of
+    rows is written instead; DIR/query.npy holds the query number of each written row."""
+    doc = res["doc"]
+    nq, k = doc.shape
+    n = res["n"].astype(np.int64)
+    arrays = {"doc": (doc, np.float64), "score": (res.get("score"), np.float32),
+              "score64": (res.get("score64"), np.float64)}
+    arrays = {name: (a, dt) for name, (a, dt) in arrays.items() if a is not None}
+    row_bytes = 2 * 8 + k * sum(np.dtype(dt).itemsize for _, dt in arrays.values())   # n + query + the k-wide arrays
+    rows = np.arange(nq)
+    if nq * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(nq, DUMP_BYTES // row_bytes, replace=False))
+    os.makedirs(d, exist_ok=True)
+    valid = np.arange(k)[None, :] < n[rows, None]
+    for name, (a, dt) in arrays.items():
+        np.save(os.path.join(d, f"{name}.npy"), np.where(valid, a[rows], 0).astype(dt))
+    np.save(os.path.join(d, "n.npy"), n[rows].astype(np.float64))
+    np.save(os.path.join(d, "query.npy"), rows.astype(np.float64))
+
+
 STRONG_MIX_QUERIES = 400_000   # side leg of the default run: C5's query mix, strong scaling, on the corpus already in HBM
 
 
-def strong_leg(m, torch, dist, index, stream, q_off_all, q_terms_all, k, rank, world, local_rank, reps=3):
+def strong_leg(m, torch, dist, index, stream, q_off_all, q_terms_all, k, rank, world, local_rank, reps):
     """Strong scaling with the gather INSIDE the clock (north_star: "per-GPU results are gathered on the host"):
     one batch, contiguous query shards (shard.shard_queries), every rank answers its shard through the C ABI from
     page-locked host buffers (canonicalise + H2D + kernels), the result rows travel GPU → GPU to rank 0 (one
@@ -248,8 +291,10 @@ def reference_arm(a, wl, k, cores, cores_how):
         oix.search_batch(sub_off, sub_terms, k, nthreads=cores, wand=True)
     t0 = time.perf_counter()
     for _ in range(a.steps):
-        oix.search_batch(sub_off, sub_terms, k, nthreads=cores, wand=True)
+        od, os_, on, _ = oix.search_batch(sub_off, sub_terms, k, nthreads=cores, wand=True)
     el = time.perf_counter() - t0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"doc": od, "score64": os_, "n": on})
     qps = n * a.steps / el
     config = {"workload": wl["desc"], "n_docs": wl["docs"], "vocab": wl["vocab"], "doc_len": wl["doclen"],
               "queries_per_gpu_per_step": nq, "terms_per_query": [wl["tmin"], wl["tmax"]], "k": k,
@@ -381,6 +426,8 @@ def main():
     ev1.record(stream)
     torch.cuda.synchronize()
     ms_total = ev0.elapsed_time(ev1)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, batch.fetch(want_f64=True))
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
@@ -402,7 +449,7 @@ def main():
     index.search_batch(q_off, q_terms, k, want_f64=False, out=out)
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    e2e_steps = max(3, min(a.steps, 10))
+    e2e_steps = a.steps
     for _ in range(e2e_steps):
         index.search_batch(q_off, q_terms, k, want_f64=False, out=out)
     torch.cuda.synchronize()
@@ -429,10 +476,10 @@ def main():
     # ---- strong scaling, gather to rank 0's host inside the clock (collective: every rank takes part) ----
     strong_obj = None
     if strong:
-        strong_obj = strong_leg(m, torch, dist, index, stream, q_all[0], q_all[1], k, rank, world, local_rank)
+        strong_obj = strong_leg(m, torch, dist, index, stream, q_all[0], q_all[1], k, rank, world, local_rank, a.steps)
     elif a.workload == "c3" and not a.no_strong:
         qs = m.synth_queries(0xB25C0DE0 + 5 + 1000, STRONG_MIX_QUERIES, wl["vocab"], 1, 8, post_off_like, 0.0)
-        strong_obj = strong_leg(m, torch, dist, index, stream, qs[0], qs[1], k, rank, world, local_rank)
+        strong_obj = strong_leg(m, torch, dist, index, stream, qs[0], qs[1], k, rank, world, local_rank, a.steps)
         if strong_obj:
             strong_obj["workload"] = (f"C5's query mix (1-8 terms, seed of configs[4]) on THIS corpus ({wl['docs']} docs): "
                                       f"one batch of {STRONG_MIX_QUERIES} queries; the 50M-doc corpus itself: --workload c5")
