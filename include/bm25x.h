@@ -197,7 +197,8 @@ void bm25x_batch_destroy(bm25x_batch *batch);
  * sealed documents.  Here the growing documents are inverted once into a second, small index handle that carries
  * the sealed statistics, so the same kernels unite their postings; a query then is two top-k searches + a merge.
  * Doc ids of the growing handle are growing ordinals (insertion order).  Re-create the handle after inserts/deletes
- * (it is as cheap as the segment is small); `maintain`/seal = build a new sealed index. */
+ * (it is as cheap as the segment is small); bm25x_index_maintain (below) folds the growing documents and the delete
+ * marks into a new sealed index, after which the growing segment starts empty again. */
 typedef struct {
     uint32_t n_docs;               /* growing documents, in VectorTuple-chain order */
     const uint32_t *doc_len;       /* [n_docs] exact lengths, or NULL: then doc_fieldnorm */
@@ -225,6 +226,56 @@ int bm25x_merge_topk(uint32_t nq, uint32_t k, const uint32_t *doc_a, const float
                      const uint16_t *payload_a, const uint32_t *n_a, const uint32_t *doc_b, const float *score_b,
                      const double *score64_b, const uint16_t *payload_b, const uint32_t *n_b, uint32_t doc_base_b,
                      uint32_t *out_doc, float *out_score, double *out_score64, uint16_t *out_payload, uint32_t *out_n);
+
+/* ---- the write side: bm25::maintain (crates/bm25/src/maintain.rs:27-311) and bm25::bulkdelete (bulkdelete.rs:20-112),
+ * called where amvacuumcleanup / ambulkdelete call them.  maintain rewrites every posting on the device: the sealed
+ * postings never cross PCIe (only per-document and per-term arrays and the growing elements do). */
+#define BM25X_DOC_NONE 0xFFFFFFFFu /* relabel entry of a document that did not survive */
+
+/* The VectorTuple chain as stored (Element.key + value), for maintain.  Exactly one of elem_key / elem_term:
+ * elem_key  [n_elem*16]  when the sealed index has term keys (keys strictly ascending inside a document);
+ * elem_term [n_elem]     when it has none (dense-ordinal surface; strictly ascending; ordinals >= n_terms(sealed)
+ *                        are new tokens and extend the vocabulary to max+1 over the surviving documents, the ones in
+ *                        between having df 0). */
+typedef struct {
+    uint32_t n_docs;
+    const uint16_t *payload;   /* [n_docs*3], or NULL = the synthetic ctid of the growing ordinal (what bm25x_growing_create
+                                  gives the same documents) */
+    const uint8_t *deleted;    /* [n_docs] VectorTuple.deleted, or NULL */
+    const uint64_t *elem_off;  /* [n_docs+1] */
+    const uint8_t *elem_key;
+    const uint32_t *elem_term;
+    const uint32_t *elem_tf;   /* != 0, < 2^24 */
+} bm25x_vectors;
+
+typedef struct {
+    double total_ms, device_ms;      /* host clock around the call; CUDA events from the first upload to the last kernel */
+    uint64_t h2d_bytes, d2h_bytes;   /* everything the call copied across PCIe */
+    uint64_t postings_in, postings_out; /* sealed postings + growing elements read; postings of the new index */
+} bm25x_maintain_stats;
+
+/* bm25::maintain: a NEW sealed index on the same device.  `sealed` is read, never modified, and stays valid; the caller
+ * swaps handles and destroys the old one.  sealed_deleted [n_docs(sealed)] or NULL; docs NULL = compaction only.
+ * relabel_out [n_docs(sealed) + docs->n_docs] or NULL: new doc id or BM25X_DOC_NONE.  Options set on `sealed`
+ * (prune, seed, seed_*, twophase, slice_min) carry over.
+ * New documents: the surviving sealed ones in doc-id order, then the surviving growing ones in chain order; payloads
+ * (ctids) carry over, doc ids do not.  Tokens: those with at least one surviving posting, ascending (keyed indexes drop
+ * the others; keyless ones keep every ordinal, with df 0).  Lengths follow the reference exactly, quirk included: a
+ * surviving SEALED document gets its number of distinct tokens (maintain.rs:337,356-360), not Σ tf; a growing one gets
+ * Σ tf (vector.rs:77-83).  So maintaining an index with some tf > 1 changes its fieldnorms and avgdl even with no
+ * deletes and no inserts.  The peak device memory is the old plus the new index.
+ * BM25X_ERR_INVALID: growing handle as `sealed`, keys for a keyless index or ordinals for a keyed one, documents that
+ * break vector.rs:39-75, BM25X_TERM_MISSING as an ordinal, no surviving document.  BM25X_ERR_UNSUPPORTED: tf >= 2^24.
+ * A failed call returns no handle and leaves `sealed` untouched. */
+int bm25x_index_maintain(const bm25x_index *sealed, const uint8_t *sealed_deleted, const bm25x_vectors *docs,
+                         bm25x_index **out, uint32_t *relabel_out, bm25x_maintain_stats *stats);
+
+/* bm25::bulkdelete for one handle (sealed or growing): deleted[d] |= payload(d) is in `dead` ([n_dead*3] ctids,
+ * ascending by (hi, lo, offset), duplicates allowed; else BM25X_ERR_INVALID).  Marks are only set, never cleared.
+ * n_marked (or NULL) = marks newly set by this call.  Searches do not consult the marks (search.rs:227-237): a deleted
+ * sealed row is returned until the next maintain, as in the reference. */
+int bm25x_bulkdelete(const bm25x_index *idx, const uint16_t *dead, uint64_t n_dead, uint8_t *deleted,
+                     uint32_t *n_marked);
 
 /* Invariants of the reference's vector types (crates/bm25/src/vector.rs:46-134): n vectors in CSR form, keys strictly
  * ascending inside a vector, term frequencies (tfs, NULL for Query-like vectors) non-zero — what Document::new / Query::new

@@ -14,6 +14,7 @@ _SO = os.environ.get("BM25X_LIBRARY") or os.path.join(_HERE, "libbm25x.so")
 MAX_K = 65535
 MAX_QUERY_TERMS = 64
 TERM_MISSING = 0xFFFFFFFF
+DOC_NONE = 0xFFFFFFFF
 
 
 class Bm25xError(RuntimeError):
@@ -45,6 +46,17 @@ class _GrowingDocs(C.Structure):
                 ("payload", C.POINTER(C.c_uint16)), ("deleted", C.POINTER(C.c_uint8)),
                 ("elem_off", C.POINTER(C.c_uint64)), ("elem_term", C.POINTER(C.c_uint32)),
                 ("elem_tf", C.POINTER(C.c_uint32))]
+
+
+class _Vectors(C.Structure):  # bm25x_vectors
+    _fields_ = [("n_docs", C.c_uint32), ("payload", C.POINTER(C.c_uint16)), ("deleted", C.POINTER(C.c_uint8)),
+                ("elem_off", C.POINTER(C.c_uint64)), ("elem_key", C.POINTER(C.c_uint8)),
+                ("elem_term", C.POINTER(C.c_uint32)), ("elem_tf", C.POINTER(C.c_uint32))]
+
+
+class MaintainStats(C.Structure):  # bm25x_maintain_stats
+    _fields_ = [("total_ms", C.c_double), ("device_ms", C.c_double), ("h2d_bytes", C.c_uint64),
+                ("d2h_bytes", C.c_uint64), ("postings_in", C.c_uint64), ("postings_out", C.c_uint64)]
 
 
 class IndexInfo(C.Structure):
@@ -118,6 +130,8 @@ def load_library():
     L.bm25x_growing_create.argtypes = [vp, C.POINTER(_GrowingDocs), C.POINTER(vp)]
     L.bm25x_search_batch_growing.argtypes = [vp, vp, C.c_uint32, u32p, u32p, C.c_uint32, u8p, u8p, u32p, f32p, f64p,
                                              u16p, u32p, C.POINTER(SearchStats)]
+    L.bm25x_index_maintain.argtypes = [vp, u8p, C.POINTER(_Vectors), C.POINTER(vp), u32p, C.POINTER(MaintainStats)]
+    L.bm25x_bulkdelete.argtypes = [vp, u16p, C.c_uint64, u8p, u32p]
     L.bm25x_merge_topk.argtypes = [C.c_uint32, C.c_uint32, u32p, f32p, f64p, u16p, u32p, u32p, f32p, f64p, u16p, u32p,
                                    C.c_uint32, u32p, f32p, f64p, u16p, u32p]
     L.bm25x_index_destroy.argtypes = [vp]
@@ -448,6 +462,55 @@ class Index:
         h = C.c_void_p()
         _check(load_library().bm25x_growing_create(self.h, C.byref(g), C.byref(h)))
         return Index._adopt(h, g.n_docs, self.n_terms)
+
+    # ---- the write side: bm25::maintain / bm25::bulkdelete ----
+    def maintain(self, deleted=None, elem_off=None, elem_key=None, elem_term=None, elem_tf=None, payload=None,
+                 growing_deleted=None):
+        """bm25x_index_maintain: a NEW sealed index from this one's surviving documents (`deleted` marks, or None) and
+        the growing documents (doc-major elem_off / elem_tf with elem_key [n_elem, 16] on a keyed index or elem_term on
+        a keyless one; None = compaction only).  Returns (Index, relabel, stats): relabel[d] = new doc id of sealed
+        document d, then of growing document g at n_docs + g, DOC_NONE for the dead.  This index is left unchanged."""
+        keep = []
+
+        def arr(a, dt, ct):
+            a = np.ascontiguousarray(a, dtype=dt)
+            keep.append(a)
+            return _p(a, ct)
+
+        v, vp = None, None
+        n_grow = 0
+        if elem_off is not None:
+            v = _Vectors()
+            v.elem_off = arr(elem_off, np.uint64, C.c_uint64)
+            v.n_docs = n_grow = len(keep[-1]) - 1
+            v.elem_tf = arr(elem_tf, np.uint32, C.c_uint32)
+            if elem_key is not None:
+                v.elem_key = arr(elem_key, np.uint8, C.c_uint8)
+            if elem_term is not None:
+                v.elem_term = arr(elem_term, np.uint32, C.c_uint32)
+            if payload is not None:
+                v.payload = arr(payload, np.uint16, C.c_uint16)
+            if growing_deleted is not None:
+                v.deleted = arr(growing_deleted, np.uint8, C.c_uint8)
+            vp = C.byref(v)
+        dl = arr(deleted, np.uint8, C.c_uint8) if deleted is not None else None
+        relabel = np.empty(self.n_docs + n_grow, np.uint32)
+        st = MaintainStats()
+        h = C.c_void_p()
+        _check(load_library().bm25x_index_maintain(self.h, dl, vp, C.byref(h), _p(relabel, C.c_uint32), C.byref(st)))
+        info = IndexInfo()
+        _check(load_library().bm25x_index_get_info(h, C.byref(info)))
+        return Index._adopt(h, info.n_docs, info.n_terms), relabel, st
+
+    def bulkdelete(self, dead, deleted=None):
+        """bm25x_bulkdelete: marks every document whose payload (ctid) is in `dead` ([n, 3] u16, sorted by (hi, lo,
+        offset)).  Returns (deleted, n_marked): the updated marks (a copy of `deleted`, or fresh zeros) and how many
+        this call set."""
+        dead = np.ascontiguousarray(dead, dtype=np.uint16).reshape(-1, 3)
+        out = np.zeros(self.n_docs, np.uint8) if deleted is None else np.array(deleted, dtype=np.uint8, copy=True)
+        n = C.c_uint32(0)
+        _check(load_library().bm25x_bulkdelete(self.h, _p(dead, C.c_uint16), len(dead), _p(out, C.c_uint8), C.byref(n)))
+        return out, n.value
 
     def search_batch_growing(self, growing, q_off, q_terms, k, allow=None, allow_growing=None, want_payload=False):
         """bm25::search over this sealed index + a growing handle (None = sealed only): ids >= n_docs are growing

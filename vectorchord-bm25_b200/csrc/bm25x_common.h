@@ -97,6 +97,7 @@ struct bm25x_index {
     int seed_max_terms = BM25X_SEED_MAX_TERMS;  // widest term-count class that runs seeded (4 or 8)
     int seed = 1;                      // 2..4-term classes, k <= BM25X_CHAMP_L, no prefilter: pools seeded from the champion lists
     int twophase = BM25X_TWOPHASE_DEFAULT;  // 2..4-term classes, k <= 224: two launches (8-byte postings, then doc ids only)
+    bool growing = false;              // made by bm25x_growing_create: scores with another index's statistics
     // page-locked staging buffer of bm25x_batch_prepare (grow-only, shared by the batches of this index)
     uint32_t *h_stage = nullptr;
     size_t h_stage_words = 0;
@@ -109,3 +110,70 @@ struct bm25x_index {
     uint32_t *eval_fn_len = nullptr;
     std::mutex eval_mutex;
 };
+
+// ---- index construction, shared by every way an index comes to life (bm25x_index.cu) ----
+
+// What the index sources (CSR columns, reference-format blocks, growing documents, maintain) share: statistics, tables,
+// allocations.
+struct BuildMeta {
+    uint32_t n_docs, n_terms;
+    const uint32_t *doc_len;
+    const uint16_t *payload;
+    const uint8_t *term_key;
+    double k1, b;
+    const uint32_t *df;  // [n_terms]
+    uint64_t n_post;
+    const uint8_t *fieldnorm = nullptr;  // when doc_len == NULL: DocumentTuple.fieldnorm per doc + JumpTuple.sum_of_document_lengths
+    uint64_t sum_len = 0;
+    // growing segment (search.rs:66-77): score with the SEALED segment's statistics instead of the index's own
+    const uint32_t *stat_df = nullptr;  // [n_terms] sealed TokenTuple.number_of_documents
+    uint32_t stat_n_docs = 0;           // sealed JumpTuple.number_of_documents
+    double stat_avgdl = 0.0;            // sealed sum_of_document_lengths / number_of_documents
+};
+
+// Allocates the index and fills everything except the postings (statistics, s0/s1 tables, fieldnorms, payload, keys,
+// padded offsets).  On failure the index is destroyed and *ixp is NULL.
+int bm25x_index_begin(const BuildMeta &m, int device, bm25x_index **ixp);
+// Bytes bm25x_index_begin + bm25x_index_finish_device copy host → device for an index of this shape.
+uint64_t bm25x_index_build_h2d_bytes(uint32_t n_docs, uint32_t n_terms);
+// After the postings are in place: pad slots, pdoc, block descriptors, per-term score bounds, champion lists.
+cudaError_t bm25x_index_finish_device(bm25x_index *ix);
+// Chunked H2D of a term-major CSR (T terms, P postings) and its scatter into ix->d.post: posting p of term t lands at
+// d_dst[t] + (p - off[t]) as {doc, tf << 8 | fieldnorm[doc]}.  d_dst: device array [T].
+cudaError_t bm25x_scatter_csr(bm25x_index *ix, uint32_t T, uint64_t P, const uint64_t *off, const uint32_t *doc,
+                              const uint32_t *tf, const uint64_t *d_dst);
+// The ctid given to document i of an index created without payloads: (block hi, block lo, offset) of a 291-tuple page.
+void bm25x_synthetic_ctid(uint32_t i, uint16_t out[3]);
+
+// Inversion of doc-major vectors (a VectorTuple chain, vector.rs:46-98) into a term-major CSR over T terms.  Documents
+// are visited in order, so every term's list comes out ascending.  Deleted documents are skipped; term_of(e) is the
+// term of element e, or BM25X_TERM_MISSING to drop it; doc_id(d) is the id document d gets in the lists.
+template <class TermOf, class DocId>
+void bm25x_invert_docs(uint32_t G, const uint64_t *elem_off, const uint8_t *deleted, const uint32_t *elem_tf, uint32_t T,
+                       TermOf term_of, DocId doc_id, std::vector<uint64_t> &off, std::vector<uint32_t> &doc,
+                       std::vector<uint32_t> &tf) {
+    off.assign((size_t)T + 1, 0);
+    for (uint32_t d = 0; d < G; d++) {
+        if (deleted && deleted[d]) continue;
+        for (uint64_t e = elem_off[d]; e < elem_off[d + 1]; e++) {
+            const uint32_t t = term_of(e);
+            if (t != BM25X_TERM_MISSING) off[(size_t)t + 1]++;
+        }
+    }
+    for (uint32_t t = 0; t < T; t++) off[(size_t)t + 1] += off[t];
+    const uint64_t P = off[T];
+    doc.assign(P ? P : 1, 0);
+    tf.assign(P ? P : 1, 0);
+    std::vector<uint64_t> cur(off.begin(), off.end() - 1);
+    for (uint32_t d = 0; d < G; d++) {
+        if (deleted && deleted[d]) continue;
+        const uint32_t id = doc_id(d);
+        for (uint64_t e = elem_off[d]; e < elem_off[d + 1]; e++) {
+            const uint32_t t = term_of(e);
+            if (t == BM25X_TERM_MISSING) continue;
+            doc[cur[t]] = id;
+            tf[cur[t]] = elem_tf[e];
+            cur[t]++;
+        }
+    }
+}

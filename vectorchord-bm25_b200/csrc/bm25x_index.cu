@@ -319,7 +319,7 @@ __global__ void __launch_bounds__(CHAMP_WARPS * 32) k_champions(const uint64_t *
     }
 }
 
-// champ_off from the host copy of df, then the lists (index_finish_device / finalize_replica; needs post, s0d, s1d)
+// champ_off from the host copy of df, then the lists (bm25x_index_finish_device / finalize_replica; needs post, s0d, s1d)
 static cudaError_t build_champions(bm25x_index *ix);
 
 template <typename T>
@@ -377,23 +377,6 @@ static cudaError_t build_champions(bm25x_index *ix) {
         }                                                                                           \
     } while (0)
 
-// What both index sources (CSR columns, reference-format blocks) share: statistics, tables, allocations.
-struct BuildMeta {
-    uint32_t n_docs, n_terms;
-    const uint32_t *doc_len;
-    const uint16_t *payload;
-    const uint8_t *term_key;
-    double k1, b;
-    const uint32_t *df;  // [n_terms]
-    uint64_t n_post;
-    const uint8_t *fieldnorm = nullptr;  // when doc_len == NULL: DocumentTuple.fieldnorm per doc + JumpTuple.sum_of_document_lengths
-    uint64_t sum_len = 0;
-    // growing segment (search.rs:66-77): score with the SEALED segment's statistics instead of the index's own
-    const uint32_t *stat_df = nullptr;  // [n_terms] sealed TokenTuple.number_of_documents
-    uint32_t stat_n_docs = 0;           // sealed JumpTuple.number_of_documents
-    double stat_avgdl = 0.0;            // sealed sum_of_document_lengths / number_of_documents
-};
-
 static int check_common(const char *who, uint32_t n_docs, const void *doc_len, double k1, double b, int device) {
     if (n_docs == 0 || n_docs == BM25X_DOC_INF || !doc_len) {
         bm25x_set_error("%s: empty or malformed corpus", who);
@@ -436,7 +419,20 @@ static void apply_env_options(bm25x_index *ix) {
     }
 }
 
-static int index_begin(const BuildMeta &m, int device, bm25x_index **ixp) {
+void bm25x_synthetic_ctid(uint32_t i, uint16_t out[3]) {
+    const uint32_t blkno = i / 291;
+    out[0] = (uint16_t)(blkno >> 16);
+    out[1] = (uint16_t)(blkno & 0xFFFF);
+    out[2] = (uint16_t)(i % 291 + 1);
+}
+
+uint64_t bm25x_index_build_h2d_bytes(uint32_t n_docs, uint32_t n_terms) {
+    const uint64_t N = n_docs, T = n_terms;
+    // post_off, blk_off, champ_off; df, s0d, s0f; s1d, s1f; fieldnorm, payload
+    return 3 * 8 * (T + 1) + (T ? (4 + 8 + 4) * T : 0) + 256 * (8 + 4) + N + 6 * N;
+}
+
+int bm25x_index_begin(const BuildMeta &m, int device, bm25x_index **ixp) {
     *ixp = nullptr;
     fn_init();
     const uint32_t N = m.n_docs, T = m.n_terms;
@@ -554,12 +550,7 @@ static int index_begin(const BuildMeta &m, int device, bm25x_index **ixp) {
         CU(cudaMemcpy(d.payload, m.payload, sizeof(uint16_t) * 3 * (size_t)N, cudaMemcpyHostToDevice));
     } else {
         std::vector<uint16_t> pl((size_t)N * 3);
-        for (uint32_t i = 0; i < N; i++) {  // synthetic ctid: (block hi, block lo, offset) of a 291-tuple page
-            uint32_t blkno = i / 291;
-            pl[(size_t)i * 3 + 0] = (uint16_t)(blkno >> 16);
-            pl[(size_t)i * 3 + 1] = (uint16_t)(blkno & 0xFFFF);
-            pl[(size_t)i * 3 + 2] = (uint16_t)(i % 291 + 1);
-        }
+        for (uint32_t i = 0; i < N; i++) bm25x_synthetic_ctid(i, &pl[(size_t)i * 3]);
         CU(cudaMemcpy(d.payload, pl.data(), sizeof(uint16_t) * pl.size(), cudaMemcpyHostToDevice));
     }
 
@@ -567,8 +558,7 @@ static int index_begin(const BuildMeta &m, int device, bm25x_index **ixp) {
     return BM25X_OK;
 }
 
-// After the postings are in place: pad slots, block descriptors, per-term score bounds.
-static cudaError_t index_finish_device(bm25x_index *ix) {
+cudaError_t bm25x_index_finish_device(bm25x_index *ix) {
     DeviceIndex &d = ix->d;
     const uint32_t T = d.n_terms;
     const uint64_t nb = d.n_blocks;
@@ -595,42 +585,45 @@ static cudaError_t index_finish_device(bm25x_index *ix) {
     return e;
 }
 
+cudaError_t bm25x_scatter_csr(bm25x_index *ix, uint32_t T, uint64_t P, const uint64_t *post_off, const uint32_t *post_doc,
+                              const uint32_t *post_tf, const uint64_t *d_dst) {
+    DeviceIndex &d = ix->d;
+    uint64_t *d_off = nullptr;
+    uint32_t *d_cdoc = nullptr, *d_ctf = nullptr;
+    const uint64_t CH = 64ull << 20;  // postings per chunk
+    uint64_t chn = std::min<uint64_t>(CH, P ? P : 1);
+    cudaError_t e1 = cudaMalloc((void **)&d_off, sizeof(uint64_t) * ((size_t)T + 1));
+    cudaError_t e2 = cudaMalloc((void **)&d_cdoc, sizeof(uint32_t) * chn);
+    cudaError_t e3 = cudaMalloc((void **)&d_ctf, sizeof(uint32_t) * chn);
+    cudaError_t e = e1 != cudaSuccess ? e1 : (e2 != cudaSuccess ? e2 : e3);
+    if (e == cudaSuccess) e = cudaMemcpy(d_off, post_off, sizeof(uint64_t) * ((size_t)T + 1), cudaMemcpyHostToDevice);
+    for (uint64_t base = 0; base < P && e == cudaSuccess; base += CH) {
+        uint64_t n = std::min<uint64_t>(CH, P - base);
+        e = cudaMemcpy(d_cdoc, post_doc + base, sizeof(uint32_t) * n, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = cudaMemcpy(d_ctf, post_tf + base, sizeof(uint32_t) * n, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) {
+            k_build_postings<<<(unsigned)((n + 255) / 256), 256>>>(d_cdoc, d_ctf, base, n, d_off, d_dst, T, d.fieldnorm,
+                                                                   d.post);
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    }
+    cudaFree(d_off);
+    cudaFree(d_cdoc);
+    cudaFree(d_ctf);
+    return e;
+}
+
 // Postings of a term-major CSR: chunked H2D of the columns + device transform to the padded AoS, then the derived arrays.
 // Destroys the index on failure.
 static int upload_csr(bm25x_index *ix, const char *who, uint32_t T, uint64_t P, const uint64_t *post_off,
                       const uint32_t *post_doc, const uint32_t *post_tf) {
-    DeviceIndex &d = ix->d;
-    // ---- postings: chunked H2D of the CSR columns + device transform to the padded AoS ----
-    {
-        uint64_t *d_off = nullptr;
-        uint32_t *d_cdoc = nullptr, *d_ctf = nullptr;
-        const uint64_t CH = 64ull << 20;  // postings per chunk
-        uint64_t chn = std::min<uint64_t>(CH, P ? P : 1);
-        cudaError_t e1 = cudaMalloc((void **)&d_off, sizeof(uint64_t) * ((size_t)T + 1));
-        cudaError_t e2 = cudaMalloc((void **)&d_cdoc, sizeof(uint32_t) * chn);
-        cudaError_t e3 = cudaMalloc((void **)&d_ctf, sizeof(uint32_t) * chn);
-        cudaError_t e = e1 != cudaSuccess ? e1 : (e2 != cudaSuccess ? e2 : e3);
-        if (e == cudaSuccess) e = cudaMemcpy(d_off, post_off, sizeof(uint64_t) * ((size_t)T + 1), cudaMemcpyHostToDevice);
-        for (uint64_t base = 0; base < P && e == cudaSuccess; base += CH) {
-            uint64_t n = std::min<uint64_t>(CH, P - base);
-            e = cudaMemcpy(d_cdoc, post_doc + base, sizeof(uint32_t) * n, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) e = cudaMemcpy(d_ctf, post_tf + base, sizeof(uint32_t) * n, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) {
-                k_build_postings<<<(unsigned)((n + 255) / 256), 256>>>(d_cdoc, d_ctf, base, n, d_off, d.post_off, T,
-                                                                       d.fieldnorm, d.post);
-                e = cudaGetLastError();
-            }
-            if (e == cudaSuccess) e = cudaDeviceSynchronize();
-        }
-        if (e == cudaSuccess) e = index_finish_device(ix);
-        cudaFree(d_off);
-        cudaFree(d_cdoc);
-        cudaFree(d_ctf);
-        if (e != cudaSuccess) {
-            bm25x_set_error("%s: posting upload failed: %s", who, cudaGetErrorString(e));
-            bm25x_index_destroy(ix);
-            return e == cudaErrorMemoryAllocation ? BM25X_ERR_OOM : BM25X_ERR_CUDA;
-        }
+    cudaError_t e = bm25x_scatter_csr(ix, T, P, post_off, post_doc, post_tf, ix->d.post_off);
+    if (e == cudaSuccess) e = bm25x_index_finish_device(ix);
+    if (e != cudaSuccess) {
+        bm25x_set_error("%s: posting upload failed: %s", who, cudaGetErrorString(e));
+        bm25x_index_destroy(ix);
+        return e == cudaErrorMemoryAllocation ? BM25X_ERR_OOM : BM25X_ERR_CUDA;
     }
     return BM25X_OK;
 }
@@ -683,7 +676,7 @@ extern "C" int bm25x_index_create(const bm25x_corpus *c, int device, bm25x_index
     for (uint32_t t = 0; t < T; t++) df[t] = (uint32_t)(c->post_off[t + 1] - c->post_off[t]);
     BuildMeta m{N, T, c->doc_len, c->payload, c->term_key, c->k1, c->b, df.data(), P};
     bm25x_index *ix = nullptr;
-    rc = index_begin(m, device, &ix);
+    rc = bm25x_index_begin(m, device, &ix);
     if (rc != BM25X_OK) return rc;
 
     rc = upload_csr(ix, "bm25x_index_create", T, P, c->post_off, c->post_doc, c->post_tf);
@@ -765,7 +758,7 @@ extern "C" int bm25x_index_create_from_blocks(const bm25x_blocks *c, int device,
     m.fieldnorm = c->doc_fieldnorm;
     m.sum_len = c->sum_doc_len;
     bm25x_index *ix = nullptr;
-    rc = index_begin(m, device, &ix);
+    rc = bm25x_index_begin(m, device, &ix);
     if (rc != BM25X_OK) return rc;
     DeviceIndex &d = ix->d;
 
@@ -795,7 +788,7 @@ extern "C" int bm25x_index_create_from_blocks(const bm25x_blocks *c, int device,
             NB, d_tbo, T, d_min, d_n, d_md, d_mt, d_doff, d_toff, d_bytes, d.post_off, d.fieldnorm, N, d.post, d_err);
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) e = index_finish_device(ix);
+    if (e == cudaSuccess) e = bm25x_index_finish_device(ix);
     uint8_t *d_wfn = nullptr;
     uint32_t *d_wtf = nullptr;
     if (c->blk_wand_fieldnorm && c->blk_wand_tf) {  // the stored per-block bounds must be those of the decoded postings
@@ -865,8 +858,7 @@ extern "C" int bm25x_growing_create(const bm25x_index *sealed, const bm25x_growi
     int rc = check_common(who, G, g->doc_len ? (const void *)g->doc_len : (const void *)g->doc_fieldnorm, sealed->k1,
                           sealed->b, sealed->device);
     if (rc != BM25X_OK) return rc;
-    // pass 1: validate the documents (vector.rs:39-75: keys strictly ascending, tf != 0) and count per-term postings
-    std::vector<uint64_t> off((size_t)T + 1, 0);
+    // validate the documents (vector.rs:39-75: keys strictly ascending, tf != 0)
     int bad = 0;
     for (uint32_t d = 0; d < G; d++) {
         const uint64_t e0 = g->elem_off[d], e1 = g->elem_off[d + 1];
@@ -886,7 +878,6 @@ extern "C" int bm25x_growing_create(const bm25x_index *sealed, const bm25x_growi
             prev = t;
             if (t >= T || sealed->h_df[t] == 0) continue;
             if (f >= (1u << 24)) bad |= 2;
-            off[(size_t)t + 1]++;
         }
     }
     if (bad & 1) {
@@ -897,27 +888,19 @@ extern "C" int bm25x_growing_create(const bm25x_index *sealed, const bm25x_growi
         bm25x_set_error("%s: term frequency >= 2^24 is not supported by the packed posting layout", who);
         return BM25X_ERR_UNSUPPORTED;
     }
+    // invert; doc ids are growing ordinals, deleted documents keep theirs
+    std::vector<uint64_t> off;
+    std::vector<uint32_t> post_doc, post_tf;
+    bm25x_invert_docs(
+        G, g->elem_off, g->deleted, g->elem_tf, T,
+        [&](uint64_t e) {
+            const uint32_t t = g->elem_term[e];
+            return t == BM25X_TERM_MISSING || t >= T || sealed->h_df[t] == 0 ? BM25X_TERM_MISSING : t;
+        },
+        [](uint32_t d) { return d; }, off, post_doc, post_tf);
     std::vector<uint32_t> df(T);
-    for (uint32_t t = 0; t < T; t++) {
-        df[t] = (uint32_t)off[(size_t)t + 1];
-        off[(size_t)t + 1] += off[t];
-    }
+    for (uint32_t t = 0; t < T; t++) df[t] = (uint32_t)(off[(size_t)t + 1] - off[t]);
     const uint64_t P = off[T];
-    // pass 2: invert (documents are visited in ascending ordinal, so every term's list comes out ascending)
-    std::vector<uint32_t> post_doc(P ? P : 1), post_tf(P ? P : 1);
-    {
-        std::vector<uint64_t> cur(off.begin(), off.end() - 1);
-        for (uint32_t d = 0; d < G; d++) {
-            if (g->deleted && g->deleted[d]) continue;
-            for (uint64_t e = g->elem_off[d]; e < g->elem_off[d + 1]; e++) {
-                const uint32_t t = g->elem_term[e];
-                if (t == BM25X_TERM_MISSING || t >= T || sealed->h_df[t] == 0) continue;
-                post_doc[cur[t]] = d;
-                post_tf[cur[t]] = g->elem_tf[e];
-                cur[t]++;
-            }
-        }
-    }
     BuildMeta m{G, T, g->doc_len, g->payload, sealed->h_keys.empty() ? nullptr : sealed->h_keys.data(), sealed->k1,
                 sealed->b, df.data(), P};
     m.fieldnorm = g->doc_fieldnorm;
@@ -925,11 +908,12 @@ extern "C" int bm25x_growing_create(const bm25x_index *sealed, const bm25x_growi
     m.stat_n_docs = sealed->d.n_docs;
     m.stat_avgdl = sealed->avgdl;
     bm25x_index *ix = nullptr;
-    rc = index_begin(m, sealed->device, &ix);
+    rc = bm25x_index_begin(m, sealed->device, &ix);
     if (rc != BM25X_OK) return rc;
     rc = upload_csr(ix, who, T, P, off.data(), post_doc.data(), post_tf.data());
     if (rc != BM25X_OK) return rc;
     ix->prune = sealed->prune;
+    ix->growing = true;
     *out = ix;
     return BM25X_OK;
 }
@@ -1074,7 +1058,7 @@ extern "C" int bm25x_index_finalize_replica(bm25x_index *ix) {
     if (ix->d.n_terms)
         BM25X_CUDA_TRY(cudaMemcpy(ix->h_df.data(), ix->d.df, sizeof(uint32_t) * ix->d.n_terms, cudaMemcpyDeviceToHost));
     if (!ix->d.champ) BM25X_CUDA_TRY(build_champions(ix));  // derived data: built here from the replicated arrays
-    {   // s1f_min from the replicated arrays (see index_begin)
+    {   // s1f_min from the replicated arrays (see bm25x_index_begin)
         std::vector<uint8_t> h_fn(ix->d.n_docs);
         float h_s1f[256];
         BM25X_CUDA_TRY(cudaMemcpy(h_fn.data(), ix->d.fieldnorm, ix->d.n_docs, cudaMemcpyDeviceToHost));
